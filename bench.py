@@ -20,6 +20,9 @@ K complete batches, first submit to last result, and nothing is skipped.  Weak s
 queries per step, the map is replicated, and (N > 1) the solved trajectories of every step are all-gathered with NCCL on a
 side stream inside the timed region.
 
+--dump-outputs DIR writes the last timed step's results (what uavmp_plan_submit returns to its caller) as DIR/<name>.npy, a fixed
+seeded sample of the queries when they exceed 64 MB, so that two builds can be compared output for output.
+
 Keys beyond the base contract: `roofline` (the search kernel: algorithmic bytes of SURVEY.md §8(d) over the timed region),
 `cpu_baseline` (bounded sample of the same workload on the host cores), `e2e` (pinned host buffers through
 uavmp_plan_submit / uavmp_plan_wait, copies inside the timed region), `clocks`, `gpu_launches`.
@@ -136,9 +139,32 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """arrays: {name: array with one row per query}; ints are written as float32, floats as float64.  Above DUMP_BYTES in all, a
+    fixed seeded sample of the rows is written, with the sampled query indices as query_index.npy."""
+    n = len(next(iter(arrays.values())))
+    row = sum(a[0].nbytes if a.dtype.kind == "f" else 4 * a[0].size for a in arrays.values())
+    if n * row > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // row, replace=False))
+        arrays = dict({k: a[idx] for k, a in arrays.items()}, query_index=idx.astype(np.float64))
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), a.astype(np.float64 if a.dtype.kind == "f" else np.float32))
+
+
 # ---------------------------------------------------------------------------------------------------------------
 # CPU path (oracle): used ONLY by the cpu_baseline leg and by --impl reference
 # ---------------------------------------------------------------------------------------------------------------
+def have_cpu_path():
+    """The CPU path solves its QPs with the reference's own OSQP (oracle/_ref), built only where the reference's sources exist."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import oracle_lib
+    return oracle_lib.have_ref()
+
+
 def cpu_plans(world, params, wl, jobs, threads):
     """Run the CPU pipeline for `jobs` = [(queries, index), ...] on `threads` host threads that pull from ONE queue in the given
     order (no barrier between steps: a long query does not idle the other threads).  Returns (wall seconds, sum of the threads'
@@ -198,6 +224,8 @@ def cpu_summary(n, wall, busy, threads):
 def run_reference(args, rank, world_size, wl):
     if rank != 0:
         return
+    if not have_cpu_path():
+        raise SystemExit("bench.py --impl reference: oracle/_ref/libosqp_ref.so (the reference's OSQP) is not built")
     import uav_motion_planning_b200 as u
     from uav_motion_planning_b200 import _lib
     world = u.make_world(*wl["map"], seed=1, map_type=wl["map_type"])  # host-only input generator (libuavmp_worldgen.so)
@@ -345,6 +373,9 @@ def run_gpu(args, rank, world_size, local_rank, wl):
     last = ring[(K - 1) % depth]
     reached = int((last["status"] == 1).sum().item())
     solved = int(last["solved"].sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"plan_status": last["status"].cpu().numpy(), "qp_solved": last["solved"].cpu().numpy(),
+                                         "coef": last["coef"].cpu().numpy()})
     bytes_a = [search_bytes(i["counters"]) for i in infos]
     pops = [i["counters"]["n_pop"] for i in infos]
     launch_ms = [i["timings"]["search_ms"] for i in infos]
@@ -405,7 +436,9 @@ def run_gpu(args, rank, world_size, local_rank, wl):
             "result_check": {"reach_end_frac_last_step": reached / B, "qp_solved_frac_last_step": solved / B,
                              "error_flags": int(np.bitwise_or.reduce(flags))},
         }
-        if world_size == 1 and not args.no_cpu:
+        if world_size == 1 and not args.no_cpu and not have_cpu_path():
+            out["cpu_baseline"] = {"unavailable": "oracle/_ref/libosqp_ref.so (the reference's OSQP) is not built"}
+        elif world_size == 1 and not args.no_cpu:
             threads = os.cpu_count() or 1
             n_s = args.cpu_sample or min(B, 16 * threads)  # ~15 s of host time at ~0.9 core-seconds per query
             jobs = lpt_jobs([batches[W]], n_s)
@@ -461,6 +494,8 @@ def run_qp_sweep(args, rank, world_size, local_rank):
                       "iters_mean": float(np.mean(iters)), "qp_iters_per_s": B * np.mean(iters) / (np.mean(ms) * 1e-3),
                       "solved_frac": float(np.mean(solved))})
     clk = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: r[k] for k in ("coef", "iters", "status", "solved")})
     base = sweep[0]
     # SURVEY.md §8(d): flops per ADMM iteration ~ 4 nnz(L) + 2 nnz(A) + 12 (n + m); order 7, S 16: nnzL 1201, nnzA 786, n 128, m 83
     nnzL, nnzA, nq, mq = 1201, 786, 128, 83
@@ -502,7 +537,10 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="queries per GPU per step (0: the configuration's own)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="queries per step in the CPU sample (0: auto)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

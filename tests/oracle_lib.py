@@ -5,6 +5,8 @@ import subprocess
 
 import numpy as np
 
+import ref_record
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 LIB = os.path.join(ORACLE_DIR, "liboracle.so")
@@ -129,8 +131,16 @@ def osqp_settings(**kw):
     return s
 
 
+_have_ref = None
+
+
 def have_ref():
-    return bool(load().oracle_have_ref())
+    """True when oracle/_ref/libosqp_ref.so (the reference's OSQP) is built; otherwise the QP calls below answer from the record
+    (tests/ref_record.py)."""
+    global _have_ref
+    if _have_ref is None:
+        _have_ref = bool(load().oracle_have_ref())
+    return _have_ref
 
 
 def info_dict(info):
@@ -146,21 +156,29 @@ def _p(a):
 
 
 def minctrl_solve(order, S, pos_1d, bound_vel, bound_acc, T, bound_jerk=None, settings=None, libm_mode=0,
-                  corridor_lo=None, corridor_hi=None, n_corridor=0):
-    """n_corridor > 0: the corridor extension (SURVEY.md §9.3) — corridor_lo / corridor_hi hold one box per segment."""
+                  corridor_lo=None, corridor_hi=None, n_corridor=0, like=None):
+    """n_corridor > 0: the corridor extension (SURVEY.md §9.3) — corridor_lo / corridor_hi hold one box per segment.
+    like: the coefficients the caller compares the result with (ref_record.call)."""
     lib = load()
     st = settings or osqp_settings()
     pos_1d, bound_vel, bound_acc, bound_jerk, T = _f(pos_1d), _f(bound_vel), _f(bound_acc), _f(bound_jerk), _f(T)
     lo, hi = _f(corridor_lo), _f(corridor_hi)
-    coef = np.zeros((order + 1) * S)
-    info = OsqpInfo()
-    lib.oracle_minctrl_solve_c.argtypes = [C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 7 + [C.POINTER(OsqpSettings), C.c_int,
-                                                                                          C.c_void_p, C.POINTER(OsqpInfo)]
-    ok = lib.oracle_minctrl_solve_c(order, S, n_corridor, _p(pos_1d), _p(bound_vel), _p(bound_acc), _p(bound_jerk), _p(T),
-                                    _p(lo), _p(hi), C.byref(st), libm_mode, _p(coef), C.byref(info))
-    if ok < 0:
-        raise RuntimeError("oracle/_ref/libosqp_ref.so is not available")
-    return ok, coef, info_dict(info)
+
+    def live():
+        coef = np.zeros((order + 1) * S)
+        info = OsqpInfo()
+        lib.oracle_minctrl_solve_c.argtypes = [C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 7 + [C.POINTER(OsqpSettings), C.c_int,
+                                                                                              C.c_void_p, C.POINTER(OsqpInfo)]
+        ok = lib.oracle_minctrl_solve_c(order, S, n_corridor, _p(pos_1d), _p(bound_vel), _p(bound_acc), _p(bound_jerk), _p(T),
+                                        _p(lo), _p(hi), C.byref(st), libm_mode, _p(coef), C.byref(info))
+        if ok < 0:
+            raise RuntimeError("oracle/_ref/libosqp_ref.so is not available")
+        return dict(ok=ok, coef=coef, info=info_dict(info))
+
+    r = ref_record.call("minctrl_solve", live if have_ref() else None,
+                        (order, S, n_corridor, pos_1d, bound_vel, bound_acc, bound_jerk, T, lo, hi, st, libm_mode),
+                        like=None if like is None else {"coef": like})
+    return r["ok"], r["coef"], r["info"]
 
 
 def minctrl_assemble(order, S, pos_1d, bound_vel, bound_acc, T, bound_jerk=None, libm_mode=0):
@@ -191,15 +209,20 @@ def osqp_solve(P_triu_csc, q, A_csc, l, u, settings=None):
     Pp, Pi, Px = _csc(P_triu_csc)
     Ap, Ai, Ax = _csc(A_csc)
     q, l, u = _f(q), _f(l), _f(u)
-    x, y = np.zeros(n), np.zeros(max(m, 1))
-    info = OsqpInfo()
-    lib.oracle_osqp_solve.argtypes = [C.c_longlong, C.c_longlong] + [C.c_void_p] * 9 + \
-        [C.POINTER(OsqpSettings), C.c_void_p, C.c_void_p, C.POINTER(OsqpInfo)]
-    rc = lib.oracle_osqp_solve(n, m, _p(Pp), _p(Pi), _p(Px), _p(q), _p(Ap), _p(Ai), _p(Ax), _p(l), _p(u),
-                               C.byref(st), _p(x), _p(y), C.byref(info))
-    if rc < 0:
-        raise RuntimeError("oracle/_ref/libosqp_ref.so is not available")
-    return x, y[:m], info_dict(info)
+
+    def live():
+        x, y = np.zeros(n), np.zeros(max(m, 1))
+        info = OsqpInfo()
+        lib.oracle_osqp_solve.argtypes = [C.c_longlong, C.c_longlong] + [C.c_void_p] * 9 + \
+            [C.POINTER(OsqpSettings), C.c_void_p, C.c_void_p, C.POINTER(OsqpInfo)]
+        rc = lib.oracle_osqp_solve(n, m, _p(Pp), _p(Pi), _p(Px), _p(q), _p(Ap), _p(Ai), _p(Ax), _p(l), _p(u),
+                                   C.byref(st), _p(x), _p(y), C.byref(info))
+        if rc < 0:
+            raise RuntimeError("oracle/_ref/libosqp_ref.so is not available")
+        return dict(x=x, y=y[:m], info=info_dict(info))
+
+    r = ref_record.call("osqp_solve", live if have_ref() else None, (n, m, Pp, Pi, Px, q, Ap, Ai, Ax, l, u, st))
+    return r["x"], r["y"], r["info"]
 
 
 def kkt_solve(P_triu_csc, A_csc, sigma, rho, rhs):
@@ -208,13 +231,17 @@ def kkt_solve(P_triu_csc, A_csc, sigma, rho, rhs):
     Pp, Pi, Px = _csc(P_triu_csc)
     Ap, Ai, Ax = _csc(A_csc)
     rhs = _f(rhs)
-    sol = np.zeros(n + m)
-    lib.oracle_osqp_kkt_solve.argtypes = [C.c_longlong, C.c_longlong] + [C.c_void_p] * 6 + \
-        [C.c_double, C.c_double, C.c_void_p, C.c_void_p]
-    rc = lib.oracle_osqp_kkt_solve(n, m, _p(Pp), _p(Pi), _p(Px), _p(Ap), _p(Ai), _p(Ax), sigma, rho, _p(rhs), _p(sol))
-    if rc:
-        raise RuntimeError(f"kkt solve failed ({rc})")
-    return sol
+
+    def live():
+        sol = np.zeros(n + m)
+        lib.oracle_osqp_kkt_solve.argtypes = [C.c_longlong, C.c_longlong] + [C.c_void_p] * 6 + \
+            [C.c_double, C.c_double, C.c_void_p, C.c_void_p]
+        rc = lib.oracle_osqp_kkt_solve(n, m, _p(Pp), _p(Pi), _p(Px), _p(Ap), _p(Ai), _p(Ax), sigma, rho, _p(rhs), _p(sol))
+        if rc:
+            raise RuntimeError(f"kkt solve failed ({rc})")
+        return dict(sol=sol)
+
+    return ref_record.call("kkt_solve", live if have_ref() else None, (n, m, Pp, Pi, Px, Ap, Ai, Ax, sigma, rho, rhs))["sol"]
 
 
 # ---- grid A* ---------------------------------------------------------------------------------------------------------
@@ -251,22 +278,29 @@ def have_astar_ref():
     return os.path.exists(os.path.join(ORACLE_DIR, "_ref", "libastar_ref.so"))
 
 
-def astar_search_reference(world, start_pt, end_pt, lambda_heu=1.0, allocated_node_num=100000, path_cap=8192):
-    """oracle/_ref/libastar_ref.so: the reference's a_star.cpp compiled unmodified against the header shims."""
-    global _astar_ref
-    if _astar_ref is None:
-        _astar_ref = C.CDLL(os.path.join(ORACLE_DIR, "_ref", "libastar_ref.so"))
-        _astar_ref.refastar_search.argtypes = [C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
-                                               C.c_double, C.c_void_p, C.c_void_p, C.POINTER(RefAstarResult), C.c_void_p, C.c_int]
+def astar_search_reference(world, start_pt, end_pt, lambda_heu=1.0, allocated_node_num=100000, path_cap=8192, like=None):
+    """oracle/_ref/libastar_ref.so: the reference's a_star.cpp compiled unmodified against the header shims (recorded result where it
+    is not built; like: a result whose path the caller compares with, see ref_record.call)."""
     occ = np.ascontiguousarray(world.occ, np.int8)
     origin, msz = _f(world.origin), _f(world.map_size)
     sp, ep = _f(start_pt), _f(end_pt)
-    res = RefAstarResult()
-    path = np.zeros((path_cap, 3))
-    _astar_ref.refastar_search(lambda_heu, allocated_node_num, occ.ctypes.data, *world.dims, _p(origin), _p(msz), world.resolution,
-                               _p(sp), _p(ep), C.byref(res), path.ctypes.data, path_cap)
-    return dict(status=res.status, use_node_num=res.use_node_num, n_path=res.n_path, lookup_digest=res.lookup_digest,
-                n_in_map_calls=res.n_in_map_calls, path=path[:min(res.n_path, path_cap)].copy())
+
+    def live():
+        global _astar_ref
+        if _astar_ref is None:
+            _astar_ref = C.CDLL(os.path.join(ORACLE_DIR, "_ref", "libastar_ref.so"))
+            _astar_ref.refastar_search.argtypes = [C.c_double, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                                   C.c_double, C.c_void_p, C.c_void_p, C.POINTER(RefAstarResult), C.c_void_p, C.c_int]
+        res = RefAstarResult()
+        path = np.zeros((path_cap, 3))
+        _astar_ref.refastar_search(lambda_heu, allocated_node_num, occ.ctypes.data, *world.dims, _p(origin), _p(msz), world.resolution,
+                                   _p(sp), _p(ep), C.byref(res), path.ctypes.data, path_cap)
+        return dict(status=res.status, use_node_num=res.use_node_num, n_path=res.n_path, lookup_digest=res.lookup_digest,
+                    n_in_map_calls=res.n_in_map_calls, path=path[:min(res.n_path, path_cap)].copy())
+
+    return ref_record.call("astar_search_reference", live if have_astar_ref() else None,
+                           (lambda_heu, allocated_node_num, occ, world.dims, origin, msz, world.resolution, sp, ep, path_cap),
+                           like=None if like is None else {"path": like["path"]})
 
 
 # ---- RRT* (SURVEY.md §8(f) row 4, second half) ----------------------------------------------------------------------------------
@@ -308,10 +342,18 @@ def rrt_search(world, start_pt, end_pt, query_seed, max_tree_node_num=100000, st
 
 
 def rrt_search_reference(world, start_pt, end_pt, query_seed, max_tree_node_num=100000, step_length=0.5, search_radius=0.5,
-                         collision_check_resolution=0.05, sample_budget=2.0, path_cap=8192):
-    """oracle/_ref/librrt_ref.so: the reference's rrt_star.cpp + kdtree.cpp compiled unmodified (shims pin the RNG and the clock)."""
-    global _rrt_ref
-    if _rrt_ref is None:
-        _rrt_ref = C.CDLL(os.path.join(ORACLE_DIR, "_ref", "librrt_ref.so"))
-    return _rrt_call(_rrt_ref.refrrt_search, world, start_pt, end_pt, query_seed, max_tree_node_num, step_length, search_radius,
-                     collision_check_resolution, sample_budget, path_cap)
+                         collision_check_resolution=0.05, sample_budget=2.0, path_cap=8192, like=None):
+    """oracle/_ref/librrt_ref.so: the reference's rrt_star.cpp + kdtree.cpp compiled unmodified (shims pin the RNG and the clock);
+    recorded result where it is not built (like: a result whose path the caller compares with, see ref_record.call)."""
+    def live():
+        global _rrt_ref
+        if _rrt_ref is None:
+            _rrt_ref = C.CDLL(os.path.join(ORACLE_DIR, "_ref", "librrt_ref.so"))
+        return _rrt_call(_rrt_ref.refrrt_search, world, start_pt, end_pt, query_seed, max_tree_node_num, step_length, search_radius,
+                         collision_check_resolution, sample_budget, path_cap)
+
+    key = (np.ascontiguousarray(world.occ, np.int8), world.dims, _f(world.origin), _f(world.map_size), world.resolution, _f(start_pt),
+           _f(end_pt), int(query_seed), max_tree_node_num, step_length, search_radius, collision_check_resolution, float(sample_budget),
+           path_cap)
+    return ref_record.call("rrt_search_reference", live if have_rrt_ref() else None, key,
+                           like=None if like is None else {"opt_path": like["opt_path"]})

@@ -2,7 +2,7 @@
 
 The chaining itself is an extension (uav_motion_planning_b200/planner.py states the rule); each half is the oracle:
 KinoOracle.search (oracle/kino_ref.cpp) and oracle_lib.minctrl_solve (restated MinimumControl assembly -> the reference's
-own OSQP in oracle/_ref).
+own OSQP in oracle/_ref, or its recorded results).
 """
 import numpy as np
 
@@ -27,8 +27,8 @@ def segment_data(path, S, seg_time, time_alloc=0, step=0.075, n_corridor=0, marg
     return path[idx], T, lo, hi
 
 
-def plan_one(orc, sp, sv, ep, ev, order, S, seg_time, settings=None, time_alloc=0, step=0.075, n_corridor=0, margin=0.0):
-    """Returns (search_status, qp_solved, coef[3, (order+1)*S], search_result)."""
+def plan_one(orc, sp, sv, ep, ev, order, S, seg_time, settings=None, time_alloc=0, step=0.075, n_corridor=0, margin=0.0, like=None):
+    """Returns (search_status, qp_solved, coef[3, (order+1)*S], search_result); like: the coef[3, ...] the caller compares with."""
     if time_alloc or n_corridor:
         r = orc.search(sp, sv, ep, ev)
         coef = np.zeros((3, (order + 1) * S))
@@ -40,7 +40,8 @@ def plan_one(orc, sp, sv, ep, ev, order, S, seg_time, settings=None, time_alloc=
             ok, c, info = oracle_lib.minctrl_solve(order, S, wp[:, ax], [sv[ax], ev[ax]], [0.0, 0.0], T,
                                                    bound_jerk=[0.0, 0.0] if order == 7 else None, settings=settings,
                                                    corridor_lo=None if lo is None else lo[:, ax],
-                                                   corridor_hi=None if hi is None else hi[:, ax], n_corridor=n_corridor)
+                                                   corridor_hi=None if hi is None else hi[:, ax], n_corridor=n_corridor,
+                                                   like=None if like is None else like[ax])
             solved &= int(ok)
             coef[ax] = c
         return r["status"], solved, coef, r
@@ -54,7 +55,8 @@ def plan_one(orc, sp, sv, ep, ev, order, S, seg_time, settings=None, time_alloc=
     solved = 1
     for ax in range(3):
         ok, c, info = oracle_lib.minctrl_solve(order, S, wp[:, ax], [sv[ax], ev[ax]], [0.0, 0.0], T,
-                                               bound_jerk=[0.0, 0.0] if order == 7 else None, settings=settings)
+                                               bound_jerk=[0.0, 0.0] if order == 7 else None, settings=settings,
+                                               like=None if like is None else like[ax])
         solved &= int(ok)
         coef[ax] = c
     return r["status"], solved, coef, r

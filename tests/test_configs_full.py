@@ -68,7 +68,7 @@ def test_config3_wall_map_12_segments_with_corridor(gpu_ctx):
     orc = oracle_lib.KinoOracle(world, ka.params)
     n_ok = n_active = 0
     for q in list(range(0, 8)) + list(range(B // 2, B // 2 + 8)):
-        st, solved, coef, _ = plan_one(orc, sp[q], sv[q], ep[q], ev[q], 7, 12, 1.0, n_corridor=2, margin=0.2)
+        st, solved, coef, _ = plan_one(orc, sp[q], sv[q], ep[q], ev[q], 7, 12, 1.0, n_corridor=2, margin=0.2, like=got["coef"][q])
         assert (st, solved) == (got["search_status"][q], got["qp_solved"][q])
         if solved:
             assert np.array_equal(coef, got["coef"][q])   # tabulated AMD order: bit-identical to the reference's OSQP

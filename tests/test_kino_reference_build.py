@@ -10,7 +10,8 @@ reference build) must agree with it on
     sequences with bit-identical states,
 
 for the golden queries (whose expected values tests/golden/kino_golden.json holds) and for > 150 random queries on both
-collision types, the code-default parameters, a pool small enough to hit "reach max node num", and the wall map.
+collision types, the code-default parameters, a pool small enough to hit "reach max node num", and the wall map.  Where
+oracle/_ref is not built, the recorded results of that build stand in for it (tests/ref_record.py).
 What stays restated (oracle/shim/Eigen/Eigen) is Eigen's floating-point association (SURVEY.md §9.1's contract).
 """
 import ctypes as C
@@ -21,14 +22,13 @@ import numpy as np
 import pytest
 
 import oracle_lib
+import ref_record
 import uav_motion_planning_b200 as u
 from uav_motion_planning_b200 import _lib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "oracle", "_ref", "libkino_ref.so")
 GOLD = json.load(open(os.path.join(ROOT, "tests", "golden", "kino_golden.json")))
-
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/libkino_ref.so not built (needs /root/reference)")
 
 
 class RefParams(C.Structure):
@@ -44,31 +44,40 @@ class RefResult(C.Structure):
 
 class ReferenceKino:
     def __init__(self, world, p):
-        self.lib = C.CDLL(LIB)
-        self.lib.refkino_create.restype = C.c_void_p
-        self.lib.refkino_create.argtypes = [C.POINTER(RefParams), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
-                                            C.c_double, C.c_void_p, C.c_int]
-        self.lib.refkino_search.argtypes = [C.c_void_p] + [C.c_void_p] * 4 + [C.POINTER(RefResult), C.c_void_p, C.c_int]
-        self.lib.refkino_destroy.argtypes = [C.c_void_p]
         rp = RefParams(p.allocated_node_num, p.collision_check_type, p.rou_time, p.lambda_heu, p.goal_tolerance, p.time_step_size,
                        p.max_velocity, p.max_accelration, p.acc_resolution, p.sample_tau, p.robot_r, p.robot_h)
         self.occ = np.ascontiguousarray(world.occ, np.int8)
         self.cloud = np.ascontiguousarray(world.cloud, np.float32)
         origin, msz = np.ascontiguousarray(world.origin, np.float64), np.ascontiguousarray(world.map_size, np.float64)
-        self.h = self.lib.refkino_create(C.byref(rp), self.occ.ctypes.data, *world.dims, origin.ctypes.data, msz.ctypes.data,
-                                         world.resolution, self.cloud.ctypes.data, len(self.cloud))
+        self.key = ref_record.digest(rp, self.occ, self.cloud, world.dims, origin, msz, world.resolution)
+        self.lib = self.h = None
+        if os.path.exists(LIB):
+            self.lib = C.CDLL(LIB)
+            self.lib.refkino_create.restype = C.c_void_p
+            self.lib.refkino_create.argtypes = [C.POINTER(RefParams), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                                C.c_double, C.c_void_p, C.c_int]
+            self.lib.refkino_search.argtypes = [C.c_void_p] + [C.c_void_p] * 4 + [C.POINTER(RefResult), C.c_void_p, C.c_int]
+            self.lib.refkino_destroy.argtypes = [C.c_void_p]
+            self.h = self.lib.refkino_create(C.byref(rp), self.occ.ctypes.data, *world.dims, origin.ctypes.data, msz.ctypes.data,
+                                             world.resolution, self.cloud.ctypes.data, len(self.cloud))
 
-    def search(self, sp, sv, ep, ev, path_cap=4096):
+    def search(self, sp, sv, ep, ev, path_cap=4096, like=None):
         sp, sv, ep, ev = (np.ascontiguousarray(a, np.float64) for a in (sp, sv, ep, ev))
-        res = RefResult()
-        path = np.zeros((path_cap, 3))
-        self.lib.refkino_search(self.h, sp.ctypes.data, sv.ctypes.data, ep.ctypes.data, ev.ctypes.data, C.byref(res),
-                                path.ctypes.data, path_cap)
-        return dict(status=res.status, use_node_num=res.use_node_num, n_path=res.n_path, path=path[:res.n_path].copy(),
-                    lookup_digest=res.lookup_digest, n_in_map_calls=res.n_in_map_calls)
+
+        def live():
+            res = RefResult()
+            path = np.zeros((path_cap, 3))
+            self.lib.refkino_search(self.h, sp.ctypes.data, sv.ctypes.data, ep.ctypes.data, ev.ctypes.data, C.byref(res),
+                                    path.ctypes.data, path_cap)
+            return dict(status=res.status, use_node_num=res.use_node_num, n_path=res.n_path, path=path[:res.n_path].copy(),
+                        lookup_digest=res.lookup_digest, n_in_map_calls=res.n_in_map_calls)
+
+        return ref_record.call("refkino_search", live if self.lib else None, (self.key, sp, sv, ep, ev, path_cap),
+                               like=None if like is None else {"path": like["path"]})
 
     def close(self):
-        self.lib.refkino_destroy(self.h)
+        if self.lib:
+            self.lib.refkino_destroy(self.h)
 
 
 def params(launch=True, **kw):
@@ -79,8 +88,8 @@ def params(launch=True, **kw):
 
 
 def agree(ref, orc, q):
-    a = ref.search(*q)
     b = orc.search(*q)
+    a = ref.search(*q, like=b)
     assert (a["status"], a["use_node_num"], a["n_path"]) == (b["status"], b["use_node_num"], b["n_path"]), (a, b)
     assert a["n_in_map_calls"] == b["n_in_map_calls"] and a["lookup_digest"] == b["lookup_digest"]
     assert np.array_equal(a["path"].view(np.uint64), b["path"].view(np.uint64))

@@ -74,7 +74,6 @@ def test_snap_extension_dimensions(S):
     assert np.linalg.matrix_rank(A) == asm["m"]
 
 
-@pytest.mark.skipif(not oracle_lib.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("case", GOLD, ids=lambda c: f"order{c['order']}_S{c['S']}")
 def test_golden_coefficients(case):
     st = oracle_lib.osqp_settings(**case["settings"])
@@ -83,13 +82,12 @@ def test_golden_coefficients(case):
                                           bound_jerk=p["bound_jerk"])
         assert sha(asm["Px"]) == p["P_sha256"] and sha(asm["Ax"]) == p["A_sha256"]
         ok, coef, info = oracle_lib.minctrl_solve(case["order"], case["S"], p["pos"], p["bound_vel"], p["bound_acc"],
-                                                  p["T"], bound_jerk=p["bound_jerk"], settings=st)
+                                                  p["T"], bound_jerk=p["bound_jerk"], settings=st, like=np.array(p["coef"]))
         assert (ok, info["status_val"], info["iter"], info["rho_updates"]) == (p["solved"], p["status_val"], p["iter"],
                                                                                p["rho_updates"])
         assert np.array_equal(coef, np.array(p["coef"]))   # same machine code, same inputs: bit-identical
 
 
-@pytest.mark.skipif(not oracle_lib.have_ref(), reason="oracle/_ref not built")
 def test_qpsolve_fixture_is_a_min_jerk_trajectory():
     # test_qpsolve.cpp:10-18 — inputs only (the reference records no outputs); check optimality conditions instead
     ok, coef, info = oracle_lib.minctrl_solve(5, 3, [1, 2, 3, 4], [0, 0], [0, 0], [1, 1, 1])

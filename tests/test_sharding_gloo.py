@@ -6,7 +6,6 @@ import socket
 import sys
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -57,7 +56,6 @@ def test_shard_ranges():
     assert shard_range(0, 0, 2) == (0, 0)
 
 
-@pytest.mark.skipif(not __import__("oracle_lib").have_ref(), reason="oracle/_ref not built")
 def test_all_gather_of_solved_trajectories_world2(tmp_path):
     import torch.multiprocessing as mp
     port = free_port()
