@@ -14,6 +14,9 @@
  *   uavmp_minctrl_solve_batch    replaces  traj_optimization::MinimumControl::solve + getCoef1d
  *                                (src/planner/traj_optimization/include/traj_optimization/minimum_control.h:34-41,
  *                                 src/planner/traj_optimization/src/minimum_control.cpp:127-202), B 1-D QPs at once
+ *   uavmp_minctrl_solve_ragged_batch  the same for problems with a different segment count each, in one call
+ *   uavmp_rrt_plan_batch         the reference's own RRTStar::search -> MinimumControl::solve flow (test_minimum_jerk.cpp:40-75),
+ *                                B queries at once
  *   uavmp_plan_batch             the search -> waypoints -> 3 x QP pipeline (an extension; the reference never
  *                                chains the two, SURVEY.md §0)
  *
@@ -193,6 +196,36 @@ int uavmp_minctrl_solve_corridor_batch(uavmp_ctx* ctx, int order, int S, int n_c
                                        const double* time_vec, const double* corridor_lo, const double* corridor_hi,
                                        const uavmp_osqp_settings* settings, double* coef, int* solved, int* osqp_status,
                                        int* iters);
+
+/* B one-dimensional MinimumControl::solve problems, problem b with its own S[b] >= 1 segments (order 5 or 7, no corridor rows).
+ * Packed inputs / outputs, problems in order: problem b's waypoints start at pos_1d[sum_{i<b}(S[i]+1)], its segment times at
+ * time_vec[sum_{i<b} S[i]], its coefficients at coef[(order+1) * sum_{i<b} S[i]].  bound_vel / bound_acc (/ bound_jerk, order 7
+ * only): B x 2.  solved / osqp_status / iters (nullable): B.  settings NULL = defaults.  Per problem, every output is bit-identical
+ * to uavmp_minctrl_solve_batch(order, S[b], 1, ...) on the same inputs: the problems whose warp workspace fits in shared memory
+ * (order 5 up to S = 103, order 7 up to S = 70) are solved by ONE grouped launch whatever their S, the others by the thread-per-problem
+ * kernel, one launch per such S (uavmp_get_timings: qp_launches). */
+int uavmp_minctrl_solve_ragged_batch(uavmp_ctx* ctx, int order, int B, const int* S, const double* pos_1d, const double* bound_vel,
+                                     const double* bound_acc, const double* bound_jerk, const double* time_vec,
+                                     const uavmp_osqp_settings* settings, double* coef, int* solved, int* osqp_status, int* iters);
+
+/* ---- the reference's RRT* -> minimum-jerk flow, batched (test_minimum_jerk.cpp:28-173 GoalCallback) ---------------------------- */
+/* For every query: RRTStar::search (as uavmp_rrt_search_batch, same parameters, seeds and results); then, if it returned REACH_END
+ * and getOptimalPath() has n >= 2 points, S = n - 1 segments with EVERY optimal-path point a waypoint, T_s = seg_time,
+ * bound_vel = (start_vel, 0), bound_acc = (0, 0) (bound_jerk = 0 for order 7), one QP per axis (test_minimum_jerk.cpp:40-75), all
+ * of the batch's QPs solved as one ragged batch (uavmp_minctrl_solve_ragged_batch) whose waypoints never leave the device.
+ * n_segments[q] = S, or 0 when no QP was posed: status 2, or REACH_END with an empty optimal path (getOptimalPath() is only written
+ * when a later sample improves the first feasible cost).  There the reference node would reuse its stale optimal_path_ (reset()
+ * does not clear it) or resize time_vec to -1; this call poses no QP instead: n_segments = 0, qp_solved = 0, no coefficients.
+ * qp_solved[q] = all three axes SOLVED.  coef_offsets (B + 1): prefix sums of 3 (order+1) S_q; query q's coefficients are axis-major
+ * [3][(order+1) S_q] (== uavmp_plan_batch's per-query layout).  Nullable: start_vel (zero), coef_offsets, osqp_status / iters (B x 3,
+ * 0 where no QP was posed).  Returns the total number of coefficients or a negative error (path longer than path_cap_nodes:
+ * UAVMP_ECAP; no map: UAVMP_ESTATE); fetch them with uavmp_rrt_plan_get_coef.  uavmp_rrt_get_paths afterwards returns the optimal
+ * paths (the waypoints).  Synchronous on the context's stream.  uavmp_get_timings: search_ms, path_ms (QP input packing), qp_ms. */
+long long uavmp_rrt_plan_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* start_vel, const double* end_pt,
+                               const uint64_t* query_seed, int order, double seg_time, const uavmp_osqp_settings* settings,
+                               int* search_status, int* n_segments, int* qp_solved, long long* coef_offsets,
+                               int* osqp_status, int* iters);
+int uavmp_rrt_plan_get_coef(uavmp_ctx* ctx, double* coef, long long cap);
 
 /* ---- pipeline: search -> waypoints -> QP (extension) ------------------------------------------------ */
 /* For every query whose search reaches the goal, S+1 waypoints are taken from the sampled path at indices

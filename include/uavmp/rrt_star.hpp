@@ -63,6 +63,22 @@ class RRTStar {
   long long searchBatch(int B, const double* start, const double* end, const uint64_t* query_seed, int* status, long long* path_offsets) {
     return uavmp_rrt_search_batch(ctx_, B, start, end, query_seed, status, nullptr, nullptr, nullptr, nullptr, path_offsets);
   }
+  // test_minimum_jerk.cpp's GoalCallback for B queries at once (uavmp_rrt_plan_batch): search, then every optimal-path point a
+  // waypoint, T_s = seg_time, one QP per axis.  n_segments[q] = S_q (0: no QP posed); query q's coefficients are
+  // coef[coef_offsets[q] .. coef_offsets[q + 1]), axis-major [3][(order+1) S_q], each axis in MinimumControl::getCoef1d's layout.
+  // start_vel may be NULL (zero).  Returns the total number of coefficients.
+  long long planMinimumJerkBatch(int B, const double* start, const double* start_vel, const double* end, const uint64_t* query_seed,
+                                 int* status, int* n_segments, int* qp_solved, std::vector<long long>& coef_offsets,
+                                 std::vector<double>& coef, int order = 5, double seg_time = 1.0,
+                                 const uavmp_osqp_settings* settings = nullptr) {
+    coef_offsets.assign((size_t)B + 1, 0);
+    long long n = uavmp_rrt_plan_batch(ctx_, B, start, start_vel, end, query_seed, order, seg_time, settings, status, n_segments, qp_solved,
+                                       coef_offsets.data(), nullptr, nullptr);
+    if (n < 0) throw std::runtime_error(uavmp_last_error(ctx_));
+    coef.resize((size_t)n);
+    if (n > 0) check(uavmp_rrt_plan_get_coef(ctx_, coef.data(), n));
+    return n;
+  }
   uavmp_ctx* context() { return ctx_; }
 
  private:

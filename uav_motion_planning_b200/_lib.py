@@ -71,6 +71,7 @@ SYMBOLS = [
     "uavmp_kino_set_path_cap", "uavmp_minctrl_solve_corridor_batch", "uavmp_plan_options_default", "uavmp_plan_submit_opt",
     "uavmp_astar_set_params", "uavmp_astar_search_batch", "uavmp_astar_get_paths",
     "uavmp_rrt_set_params", "uavmp_rrt_sample_seed", "uavmp_rrt_search_batch", "uavmp_rrt_get_paths",
+    "uavmp_minctrl_solve_ragged_batch", "uavmp_rrt_plan_batch", "uavmp_rrt_plan_get_coef",
 ]
 
 WORLDGEN_SYMBOLS = ["uavmp_mapgen_params_default", "uavmp_mapgen_cloud", "uavmp_grid_inflate_host"]
@@ -177,6 +178,10 @@ def load():
     lib.uavmp_rrt_search_batch.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.uavmp_rrt_search_batch.restype = C.c_longlong
     lib.uavmp_rrt_get_paths.argtypes = [vp, vp, C.c_longlong]
+    lib.uavmp_minctrl_solve_ragged_batch.argtypes = [vp, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp, C.POINTER(OsqpSettings), vp, vp, vp, vp]
+    lib.uavmp_rrt_plan_batch.argtypes = [vp, C.c_int, vp, vp, vp, vp, C.c_int, C.c_double, C.POINTER(OsqpSettings), vp, vp, vp, vp, vp, vp]
+    lib.uavmp_rrt_plan_batch.restype = C.c_longlong
+    lib.uavmp_rrt_plan_get_coef.argtypes = [vp, vp, C.c_longlong]
     lib.uavmp_kino_set_profile.argtypes = [vp, C.c_int]
     lib.uavmp_kino_get_profile.argtypes = [vp, vp, vp, C.c_int, ip]
     _lib = lib

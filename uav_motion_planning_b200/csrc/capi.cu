@@ -154,7 +154,7 @@ void uavmp_ctx_destroy(uavmp_ctx* ctx) {
   cudaStreamSynchronize(ctx->stream);
   void* ptrs[] = {ctx->d_kparams, ctx->d_lattice, ctx->d_occ, ctx->d_flags, ctx->d_tmp, ctx->d_cloud, ctx->d_cell_start,
                   ctx->d_pts, ctx->d_map, ctx->d_arena_mem, ctx->d_arenas, ctx->d_arena_busy, ctx->d_path_packed,
-                  ctx->qp_scr.ws, ctx->d_qp_in, ctx->d_qp_out, ctx->d_qp_int, ctx->d_phase, ctx->d_query_cycles,
+                  ctx->qp_scr.ws, ctx->qp_scr.tab, ctx->qp_scr.tmp, ctx->d_qp_in, ctx->d_qp_out, ctx->d_qp_int, ctx->d_phase, ctx->d_query_cycles,
                   ctx->d_flags_pad, ctx->d_b3f};
   for (void* p : ptrs) if (p) cudaFree(p);
   for (PlanSlot& sl : ctx->slots) {
@@ -476,6 +476,85 @@ int uavmp_minctrl_solve_corridor_batch(uavmp_ctx* ctx, int order, int S, int Kc,
   cudaEventElapsedTime(&ctx->tm.total_ms, ctx->ev[0], ctx->ev[3]);
   ctx->tm.qp_launches = launches;
   return UAVMP_OK;
+}
+
+int uavmp_minctrl_solve_ragged_batch(uavmp_ctx* ctx, int order, int B, const int* S, const double* pos_1d, const double* bound_vel,
+                                     const double* bound_acc, const double* bound_jerk, const double* time_vec,
+                                     const uavmp_osqp_settings* settings, double* coef, int* solved, int* osqp_status, int* iters) {
+  if (!ctx || B <= 0 || !S || !pos_1d || !bound_vel || !bound_acc || !time_vec || !coef) return UAVMP_EINVAL;
+  if (order != 5 && order != 7) return uavmp_fail(ctx, UAVMP_EINVAL, "order must be 5 (jerk) or 7 (snap)");
+  if (order == 7 && !bound_jerk) return uavmp_fail(ctx, UAVMP_EINVAL, "order 7 needs bound_jerk");
+  long long sumS = 0;
+  for (int b = 0; b < B; b++) {
+    if (S[b] < 1) return uavmp_fail(ctx, UAVMP_EINVAL, "S[%d] = %d: every problem needs at least one segment", b, S[b]);
+    sumS += S[b];
+  }
+  uavmp_osqp_settings def;
+  if (!settings) { uavmp_osqp_settings_default(&def); settings = &def; }
+  if (settings->max_iter <= 0 || settings->check_termination < 0 || settings->scaling < 0)
+    return uavmp_fail(ctx, UAVMP_EINVAL, "bad OSQP settings");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  const size_t n_pos = (size_t)(sumS + B), n_coef = (size_t)(order + 1) * sumS;
+  int r = ensure_bytes(ctx, (void**)&ctx->d_qp_in, &ctx->qp_in_bytes, (n_pos + 6 * (size_t)B + sumS) * sizeof(double)); if (r) return r;
+  r = ensure_bytes(ctx, (void**)&ctx->d_qp_out, &ctx->qp_out_bytes, n_coef * sizeof(double)); if (r) return r;
+  r = ensure_bytes(ctx, (void**)&ctx->d_qp_int, &ctx->qp_int_bytes, (size_t)B * 3 * sizeof(int)); if (r) return r;
+  double* d_pos = ctx->d_qp_in; double* d_bv = d_pos + n_pos; double* d_ba = d_bv + 2 * (size_t)B; double* d_bj = d_ba + 2 * (size_t)B;
+  double* d_T = d_bj + 2 * (size_t)B;
+  int* d_solved = ctx->d_qp_int; int* d_stat = d_solved + B; int* d_it = d_stat + B;
+  cudaEventRecord(ctx->ev[0], st);
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(d_pos, pos_1d, n_pos * sizeof(double), cudaMemcpyHostToDevice, st));
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(d_bv, bound_vel, (size_t)B * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(d_ba, bound_acc, (size_t)B * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (order == 7) UAVMP_CUDA(ctx, cudaMemcpyAsync(d_bj, bound_jerk, (size_t)B * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(d_T, time_vec, (size_t)sumS * sizeof(double), cudaMemcpyHostToDevice, st));
+  cudaEventRecord(ctx->ev[1], st);
+  QpRaggedIo io;
+  io.pos = d_pos; io.bv = d_bv; io.ba = d_ba; io.bj = order == 7 ? d_bj : nullptr; io.T = d_T;
+  io.coef = ctx->d_qp_out; io.solved = d_solved; io.status = d_stat; io.iters = d_it; io.seg_off = nullptr; io.order = order;
+  int launches = 0, aux = 0;
+  r = qp_solve_ragged_dev(ctx, st, ctx->qp_scr, order, B, S, io, settings, &launches, &aux, nullptr, nullptr);
+  if (r) return r;
+  cudaEventRecord(ctx->ev[2], st);
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(coef, ctx->d_qp_out, n_coef * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (solved) UAVMP_CUDA(ctx, cudaMemcpyAsync(solved, d_solved, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  if (osqp_status) UAVMP_CUDA(ctx, cudaMemcpyAsync(osqp_status, d_stat, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  if (iters) UAVMP_CUDA(ctx, cudaMemcpyAsync(iters, d_it, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  cudaEventRecord(ctx->ev[3], st);
+  UAVMP_CUDA(ctx, cudaStreamSynchronize(st));
+  memset(&ctx->tm, 0, sizeof(ctx->tm));
+  cudaEventElapsedTime(&ctx->tm.h2d_ms, ctx->ev[0], ctx->ev[1]);
+  cudaEventElapsedTime(&ctx->tm.qp_ms, ctx->ev[1], ctx->ev[2]);
+  cudaEventElapsedTime(&ctx->tm.d2h_ms, ctx->ev[2], ctx->ev[3]);
+  cudaEventElapsedTime(&ctx->tm.total_ms, ctx->ev[0], ctx->ev[3]);
+  ctx->tm.qp_launches = launches;
+  ctx->tm.aux_launches = aux;
+  return UAVMP_OK;
+}
+
+// ---- RRT* -> minimum jerk (test_minimum_jerk.cpp GoalCallback, batched) ------------------------------------------------------
+long long uavmp_rrt_plan_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* start_vel, const double* end_pt,
+                               const uint64_t* query_seed, int order, double seg_time, const uavmp_osqp_settings* settings,
+                               int* search_status, int* n_segments, int* qp_solved, long long* coef_offsets, int* osqp_status,
+                               int* iters) {
+  if (!ctx || B <= 0 || !start_pt || !end_pt || !query_seed || !search_status || !n_segments || !qp_solved) return UAVMP_EINVAL;
+  if (order != 5 && order != 7) return uavmp_fail(ctx, UAVMP_EINVAL, "order must be 5 (jerk) or 7 (snap)");
+  if (!(seg_time > 0.0)) return uavmp_fail(ctx, UAVMP_EINVAL, "seg_time must be > 0");
+  uavmp_osqp_settings def;
+  if (!settings) { uavmp_osqp_settings_default(&def); settings = &def; }
+  if (settings->max_iter <= 0 || settings->check_termination < 0 || settings->scaling < 0)
+    return uavmp_fail(ctx, UAVMP_EINVAL, "bad OSQP settings");
+  cudaSetDevice(ctx->device);
+  if (!ctx->have_map) return uavmp_fail(ctx, UAVMP_ESTATE, "uavmp_map_set has not been called");
+  drain_all(ctx);
+  return rrt_plan_batch(ctx, B, start_pt, start_vel, end_pt, query_seed, order, seg_time, settings, search_status, n_segments, qp_solved,
+                        coef_offsets, osqp_status, iters);
+}
+
+int uavmp_rrt_plan_get_coef(uavmp_ctx* ctx, double* coef, long long cap) {
+  if (!ctx || !coef) return UAVMP_EINVAL;
+  cudaSetDevice(ctx->device);
+  return rrt_plan_get_coef(ctx, coef, cap);
 }
 
 // ---- pipeline ---------------------------------------------------------------------------------------------

@@ -20,12 +20,16 @@
 // minimum-degree order and agree to rounding only (the parity gate there is 1e-5 relative + identical status / iterations).
 //
 // Three executions of the same restatement: qp_solve_kernel (one thread per problem, batch-interleaved workspace),
-// qp_solve_warp_kernel (one warp per problem, workspace in shared memory) and — for the search -> QP pipeline — the same
-// warp body called from inside kino_search_kernel by the CTA that finished the query (kino_kernel.cu: qp_round).
+// qp_solve_warp_kernel (one warp per problem, workspace in shared memory; qp_solve_grouped_kernel runs the same warp body over
+// problems of different S in one launch) and — for the search -> QP pipeline — the same warp body called from inside
+// kino_search_kernel by the CTA that finished the query (kino_kernel.cu: qp_round).
 #include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <string.h>
 
+#include <algorithm>
+#include <functional>
 #include <vector>
 
 #include "fpmath.h"
@@ -78,6 +82,79 @@ static int qpw_warps_per_cta(const QpPlanDev& pl, int B) {
   if (w1 > 16) w1 = 16;
   if (w2 > 8) w2 = 8;
   return (2 * w2 >= w1) ? w2 : w1;
+}
+
+// ---- K2g: grouped warp-per-problem kernel — one launch for problems of different S (ragged batches) ------------------------------
+// A chunk is up to `wps` problems of one group (one S, one plan).  One persistent CTA per SM pulls chunks from a global counter,
+// stages the group's plan view and index block, and its warps run qp_warp_solve_one unchanged: the same body with the same plan as
+// qp_solve_warp_kernel, so every problem's result is bit-identical to a per-S launch.  Only the scheduling differs.
+struct QpChunkGroup {
+  QpPlanDev pl;
+  const int* pid;  // the group's problems (indices into the ragged batch)
+  int count;       // problems in the group
+  int wps;         // problems per chunk = warp workspaces that fit next to the index block
+  int chunk0;      // first chunk of the group (groups are stored in processing order)
+};
+
+__global__ void qp_solve_grouped_kernel(const QpChunkGroup* __restrict__ groups, int n_groups, int n_chunks, QpRaggedIo r,
+                                        uavmp_osqp_settings S, int* next_chunk) {
+  extern __shared__ __align__(16) double qpg_sm[];
+  __shared__ __align__(16) QpPlanDev s_pl;
+  __shared__ int s_chunk, s_group;
+  static_assert(sizeof(QpPlanDev) % 4 == 0, "plan view copied as words");
+  const int warp = threadIdx.x >> 5;
+  for (;;) {
+    if (threadIdx.x == 0) {
+      const int c = atomicAdd(next_chunk, 1);
+      int lo = 0, hi = n_groups - 1;  // last group with chunk0 <= c
+      while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (groups[mid].chunk0 <= c) lo = mid; else hi = mid - 1; }
+      s_chunk = c; s_group = lo;
+    }
+    __syncthreads();
+    const int c = s_chunk;
+    if (c >= n_chunks) return;  // uniform: the whole CTA leaves
+    const QpChunkGroup& G = groups[s_group];
+    for (int i = threadIdx.x; i < (int)(sizeof(QpPlanDev) / 4); i += blockDim.x)
+      reinterpret_cast<uint32_t*>(&s_pl)[i] = reinterpret_cast<const uint32_t*>(&G.pl)[i];
+    const int wps = G.wps, ws_warp = G.pl.ws_warp, n_sidx = G.pl.n_sidx;
+    unsigned short* sx = reinterpret_cast<unsigned short*>(qpg_sm + (size_t)wps * ws_warp);
+    const uint32_t* gsx = reinterpret_cast<const uint32_t*>(G.pl.Sidx);
+    for (int i = threadIdx.x; i < n_sidx / 2; i += blockDim.x) reinterpret_cast<uint32_t*>(sx)[i] = gsx[i];
+    __syncthreads();
+    const int j = (c - G.chunk0) * wps + warp;
+    if (warp < wps && j < G.count) {
+      const int p = G.pid[j];
+      const long long so = r.seg_off[p];
+      QpIo io;
+      io.pos = r.pos + so + p; io.bv = r.bv + 2 * (size_t)p; io.ba = r.ba + 2 * (size_t)p; io.bj = r.bj + 2 * (size_t)p;
+      io.T = r.T + so; io.lo = nullptr; io.hi = nullptr;
+      io.coef = r.coef + (size_t)(r.order + 1) * so; io.solved = r.solved + p; io.status = r.status + p; io.iters = r.iters + p;
+      io.B = 1; io.stride = 0;
+      qp_warp_solve_one(s_pl, io, S, qpg_sm + (size_t)warp * ws_warp, 0, sx);
+    }
+    __syncthreads();  // the next chunk may restage the plan and the index block
+  }
+}
+
+// problems of a group whose warp workspace does not fit in shared memory: copied to / from a contiguous batch for qp_solve_kernel
+__global__ void k_ragged_gather(QpRaggedIo r, const int* pid, int S, double* pos, double* bv, double* ba, double* bj, double* T) {
+  const int j = blockIdx.x, p = pid[j];
+  const long long so = r.seg_off[p];
+  for (int i = threadIdx.x; i <= S; i += blockDim.x) pos[(size_t)j * (S + 1) + i] = r.pos[so + p + i];
+  for (int i = threadIdx.x; i < S; i += blockDim.x) T[(size_t)j * S + i] = r.T[so + i];
+  if (threadIdx.x < 2) {
+    bv[2 * j + threadIdx.x] = r.bv[2 * (size_t)p + threadIdx.x];
+    ba[2 * j + threadIdx.x] = r.ba[2 * (size_t)p + threadIdx.x];
+    bj[2 * j + threadIdx.x] = r.bj[2 * (size_t)p + threadIdx.x];
+  }
+}
+
+__global__ void k_ragged_scatter(QpRaggedIo r, const int* pid, int n, const double* coef, const int* solved, const int* status,
+                                 const int* iters) {
+  const int j = blockIdx.x, p = pid[j];
+  double* out = r.coef + (size_t)(r.order + 1) * r.seg_off[p];
+  for (int i = threadIdx.x; i < n; i += blockDim.x) out[i] = coef[(size_t)j * n + i];
+  if (threadIdx.x == 0) { r.solved[p] = solved[j]; r.status[p] = status[j]; r.iters[p] = iters[j]; }
 }
 
 // ---- pipeline glue: waypoints from the searched paths, outputs back to per-plan layout --------------------------------------
@@ -248,5 +325,115 @@ int qp_scatter_plan_outputs(uavmp_ctx* ctx, PlanSlot& sl, int B, int order, int 
   const int n = (order + 1) * S;
   k_scatter_plan<<<B, 128, 0, sl.stream>>>(B, n, sl.d_status, d_solved3, d_coef3, d_qp_solved, d_coef);
   UAVMP_CUDA(ctx, cudaGetLastError());
+  return UAVMP_OK;
+}
+
+// ---- ragged batches: problems with different S in one grouped launch ------------------------------------------------------------
+// Groups whose warp workspace fits in shared memory (qpw_warps_per_cta != 0, the same test qp_solve_batch_dev applies) are cut into
+// chunks of W_S problems, W_S = warp workspaces that fit next to the group's index block in one 226 KB CTA (at most 16), and solved
+// by ONE qp_solve_grouped_kernel launch, longest S first.  The other groups run through qp_solve_batch_dev's thread-per-problem
+// kernel, one launch per S, exactly as uavmp_minctrl_solve_batch runs them.  UAVMP_QP_RAGGED_CTAS=2: two 112 KB CTAs per SM
+// instead (used only when every grouped S fits; measured, see DESIGN.md §4); UAVMP_QP_RAGGED_ASC=1: chunks by increasing S.
+int qp_solve_ragged_dev(uavmp_ctx* ctx, cudaStream_t st, QpScratch& scr, int order, int B, const int* S_host, QpRaggedIo r,
+                        const uavmp_osqp_settings* settings, int* qp_launches, int* aux_launches, int* n_groups_out, int* n_thread_out) {
+  if (settings->max_iter <= 0 || settings->check_termination < 0 || settings->scaling < 0)
+    return uavmp_fail(ctx, UAVMP_EINVAL, "bad OSQP settings");
+  // problems by S (counting sort over the distinct values)
+  std::vector<int> Svals(S_host, S_host + B);
+  std::sort(Svals.begin(), Svals.end());
+  Svals.erase(std::unique(Svals.begin(), Svals.end()), Svals.end());
+  const bool ascending = getenv("UAVMP_QP_RAGGED_ASC") != nullptr;
+  if (!ascending) std::reverse(Svals.begin(), Svals.end());
+  const int nS = (int)Svals.size();
+  std::vector<QpPlan*> plans(nS);
+  std::vector<int> cnt(nS, 0), start(nS + 1, 0), wps(nS, 0);
+  for (int g = 0; g < nS; g++) {
+    plans[g] = get_plan(ctx, order, Svals[g], 0);
+    if (!plans[g]) return uavmp_fail(ctx, UAVMP_ECUDA, "cannot build the QP plan");
+  }
+  auto group_of = [&](int S) {
+    return ascending ? (int)(std::lower_bound(Svals.begin(), Svals.end(), S) - Svals.begin())
+                     : (int)(std::lower_bound(Svals.begin(), Svals.end(), S, std::greater<int>()) - Svals.begin());
+  };
+  std::vector<int> grp(B);
+  for (int p = 0; p < B; p++) cnt[grp[p] = group_of(S_host[p])]++;
+  for (int g = 0; g < nS; g++) start[g + 1] = start[g] + cnt[g];
+  // shared-memory budget of one CTA
+  bool two = getenv("UAVMP_QP_RAGGED_CTAS") && atoi(getenv("UAVMP_QP_RAGGED_CTAS")) == 2;
+  auto fit = [](const QpPlanDev& pl, size_t budget, int cap) {
+    const size_t per = (size_t)pl.ws_warp * sizeof(double), idx = (size_t)pl.n_sidx * sizeof(unsigned short);
+    if (pl.n_sidx == 0 || per + idx > budget) return 0;
+    return std::min(cap, (int)((budget - idx) / per));
+  };
+  for (int g = 0; g < nS; g++)
+    if (qpw_warps_per_cta(plans[g]->dev, cnt[g]) && two && fit(plans[g]->dev, 112 * 1024, 8) == 0) two = false;
+  const size_t budget = two ? 112 * 1024 : 226 * 1024;
+  // host image of the table: counter | groups | seg_off[B] | pid[B]
+  std::vector<long long> seg_off(B);
+  long long so = 0;
+  for (int p = 0; p < B; p++) { seg_off[p] = so; so += S_host[p]; }
+  const size_t o_groups = 256, o_seg = o_groups + ((sizeof(QpChunkGroup) * nS + 255) & ~(size_t)255), o_pid = o_seg + (size_t)B * 8;
+  const size_t tab_bytes = o_pid + (size_t)B * 4;
+  int r0 = ensure_bytes(ctx, &scr.tab, &scr.tab_bytes, tab_bytes);
+  if (r0) return r0;
+  char* d_tab = (char*)scr.tab;
+  std::vector<char> img(tab_bytes, 0);
+  int* pid = (int*)(img.data() + o_pid);
+  {
+    std::vector<int> fill(start.begin(), start.end() - 1);
+    for (int p = 0; p < B; p++) pid[fill[grp[p]]++] = p;
+  }
+  memcpy(img.data() + o_seg, seg_off.data(), (size_t)B * 8);
+  std::vector<QpChunkGroup> tab;
+  std::vector<int> thread_groups;
+  int n_chunks = 0, max_w = 0;
+  size_t smem = 0;
+  for (int g = 0; g < nS; g++) {
+    const QpPlanDev& pl = plans[g]->dev;
+    const int w = qpw_warps_per_cta(pl, cnt[g]) ? fit(pl, budget, two ? 8 : 16) : 0;
+    if (w == 0) { thread_groups.push_back(g); continue; }
+    QpChunkGroup G;
+    G.pl = pl; G.pid = (const int*)(d_tab + o_pid) + start[g]; G.count = cnt[g]; G.wps = w; G.chunk0 = n_chunks;
+    n_chunks += (cnt[g] + w - 1) / w;
+    max_w = std::max(max_w, w);
+    smem = std::max(smem, (size_t)w * pl.ws_warp * sizeof(double) + (size_t)pl.n_sidx * sizeof(unsigned short));
+    tab.push_back(G);
+  }
+  if (!tab.empty()) memcpy(img.data() + o_groups, tab.data(), sizeof(QpChunkGroup) * tab.size());
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(d_tab, img.data(), tab_bytes, cudaMemcpyHostToDevice, st));
+  r.seg_off = (const long long*)(d_tab + o_seg);
+  if (!r.bj) r.bj = r.ba;
+  int qp_l = 0, aux_l = 0;
+  if (!tab.empty()) {
+    UAVMP_CUDA(ctx, cudaFuncSetAttribute(qp_solve_grouped_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int grid = std::min(n_chunks, ctx->sm_count * (two ? 2 : 1));
+    qp_solve_grouped_kernel<<<grid, 32 * max_w, smem, st>>>((const QpChunkGroup*)(d_tab + o_groups), (int)tab.size(), n_chunks, r,
+                                                           *settings, (int*)d_tab);
+    UAVMP_CUDA(ctx, cudaGetLastError());
+    qp_l++;
+  }
+  for (int g : thread_groups) {
+    const int S = Svals[g], nb = cnt[g], n = (order + 1) * S;
+    const size_t nd = (size_t)nb * ((S + 1) + 6 + S + n), ni = (size_t)nb * 3;
+    int rr = ensure_bytes(ctx, &scr.tmp, &scr.tmp_bytes, nd * sizeof(double) + ni * sizeof(int));
+    if (rr) return rr;
+    double* pos = (double*)scr.tmp; double* bv = pos + (size_t)nb * (S + 1); double* ba = bv + 2 * (size_t)nb; double* bj = ba + 2 * (size_t)nb;
+    double* T = bj + 2 * (size_t)nb; double* coef = T + (size_t)nb * S;
+    int* solved = (int*)(coef + (size_t)nb * n); int* status = solved + nb; int* iters = status + nb;
+    const int* gp = (const int*)(d_tab + o_pid) + start[g];
+    k_ragged_gather<<<nb, 128, 0, st>>>(r, gp, S, pos, bv, ba, bj, T);
+    UAVMP_CUDA(ctx, cudaGetLastError());
+    int l = 0;
+    rr = qp_solve_batch_dev(ctx, st, scr, &l, order, S, 0, nb, pos, bv, ba, order == 7 ? bj : nullptr, T, nullptr, nullptr, settings, coef,
+                            solved, status, iters);
+    if (rr) return rr;
+    k_ragged_scatter<<<nb, 128, 0, st>>>(r, gp, n, coef, solved, status, iters);
+    UAVMP_CUDA(ctx, cudaGetLastError());
+    qp_l += l; aux_l += 2;
+  }
+  if (qp_launches) *qp_launches = qp_l;
+  if (aux_launches) *aux_launches = aux_l;
+  if (n_groups_out) *n_groups_out = nS;
+  if (n_thread_out) *n_thread_out = (int)thread_groups.size();
   return UAVMP_OK;
 }

@@ -424,6 +424,11 @@ struct RrtState {
   long long *d_nsamples = nullptr, *d_offsets = nullptr;
   double *d_goal_g = nullptr, *d_path_stage = nullptr, *d_packed = nullptr;
   long long packed_cap = 0, last_total = 0;
+  // uavmp_rrt_plan_batch: ragged QP inputs / coefficients, per-problem results, per-QP-query packing table
+  double* d_plan = nullptr; size_t plan_bytes = 0;
+  int* d_plan_i = nullptr; size_t plan_i_bytes = 0;
+  long long* d_plan_q = nullptr; size_t plan_q_bytes = 0;
+  double* d_plan_coef = nullptr; long long plan_total = -1;
 };
 
 static void rrt_free_batch(RrtState* a) {
@@ -438,6 +443,9 @@ static void rrt_free(RrtState* a) {
   if (a->mem) cudaFree(a->mem);
   if (a->d_arenas) cudaFree(a->d_arenas);
   if (a->d_packed) cudaFree(a->d_packed);
+  if (a->d_plan) cudaFree(a->d_plan);
+  if (a->d_plan_i) cudaFree(a->d_plan_i);
+  if (a->d_plan_q) cudaFree(a->d_plan_q);
   *a = RrtState();
 }
 void rrt_destroy(uavmp_ctx* ctx) {
@@ -511,10 +519,25 @@ __global__ void k_rrt_pack(const double* stage, const int* n_path, const long lo
   double* dst = out + offsets[q] * 3;
   for (int i = threadIdx.x; i < 3 * n; i += blockDim.x) dst[i] = src[i];
 }
+// QP inputs of uavmp_rrt_plan_batch, straight from the optimal paths: query k of the QP set (source query kq[3k], S = kq[3k+1]
+// segments, sum of S over the QP queries before it kq[3k+2] = Q) owns problems 3k + axis of the ragged batch (QpRaggedIo layout:
+// segment offset 3 Q + axis S); every optimal-path point is a waypoint and every T_s = seg_time
+__global__ void k_rrt_plan_inputs(const long long* kq, const double* stage, int path_cap, double seg_time, double* pos, double* T) {
+  const int k = blockIdx.x;
+  const long long q = kq[3 * k], S = kq[3 * k + 1], Q = kq[3 * k + 2];
+  const double* path = stage + (size_t)q * path_cap * 3;
+  for (int ax = 0; ax < 3; ax++) {
+    const long long p = 3 * (long long)k + ax, so = 3 * Q + ax * S;
+    for (long long i = threadIdx.x; i <= S; i += blockDim.x) pos[so + p + i] = path[3 * i + ax];
+    for (long long i = threadIdx.x; i < S; i += blockDim.x) T[so + i] = seg_time;
+  }
+}
 }  // namespace
 
-long long rrt_search_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* end_pt, const uint64_t* query_seed, int* status,
-                           int* use_node_num, long long* n_samples, double* goal_g_cost, uint64_t* tree_digest, long long* path_offsets) {
+// the search itself, shared by uavmp_rrt_search_batch and uavmp_rrt_plan_batch: inputs up, kernel, path offsets, the post-search
+// sync with its capacity checks, and the packing of the optimal paths (what uavmp_rrt_get_paths returns).  Returns the total number
+// of path points or an error; per-query results stay on the device.
+static long long rrt_search_run(uavmp_ctx* ctx, int B, const double* start_pt, const double* end_pt, const uint64_t* query_seed) {
   int r = rrt_ensure(ctx, B);
   if (r) return r;
   RrtState& a = *ctx->rrt;
@@ -556,6 +579,16 @@ long long rrt_search_batch(uavmp_ctx* ctx, int B, const double* start_pt, const 
     a.packed_cap = cap;
   }
   if (total > 0) k_rrt_pack<<<B, 128, 0, st>>>(a.d_path_stage, a.d_nopt, a.d_offsets, a.path_cap, a.d_packed);
+  a.last_total = total;
+  return total;
+}
+
+long long rrt_search_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* end_pt, const uint64_t* query_seed, int* status,
+                           int* use_node_num, long long* n_samples, double* goal_g_cost, uint64_t* tree_digest, long long* path_offsets) {
+  const long long total = rrt_search_run(ctx, B, start_pt, end_pt, query_seed);
+  if (total < 0) return total;
+  RrtState& a = *ctx->rrt;
+  cudaStream_t st = ctx->stream;
   UAVMP_CUDA(ctx, cudaMemcpyAsync(status, a.d_status, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
   if (use_node_num) UAVMP_CUDA(ctx, cudaMemcpyAsync(use_node_num, a.d_use, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
   if (n_samples) UAVMP_CUDA(ctx, cudaMemcpyAsync(n_samples, a.d_nsamples, (size_t)B * sizeof(long long), cudaMemcpyDeviceToHost, st));
@@ -563,7 +596,6 @@ long long rrt_search_batch(uavmp_ctx* ctx, int B, const double* start_pt, const 
   if (tree_digest) UAVMP_CUDA(ctx, cudaMemcpyAsync(tree_digest, a.d_digest, (size_t)B * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
   if (path_offsets) UAVMP_CUDA(ctx, cudaMemcpyAsync(path_offsets, a.d_offsets, (size_t)(B + 1) * sizeof(long long), cudaMemcpyDeviceToHost, st));
   UAVMP_CUDA(ctx, cudaStreamSynchronize(st));
-  a.last_total = total;
   return total;
 }
 
@@ -572,6 +604,118 @@ int rrt_get_paths(uavmp_ctx* ctx, double* path_xyz, long long cap_points) {
   RrtState& a = *ctx->rrt;
   if (cap_points < a.last_total) return uavmp_fail(ctx, UAVMP_ECAP, "path buffer too small");
   if (a.last_total > 0) UAVMP_CUDA(ctx, cudaMemcpyAsync(path_xyz, a.d_packed, (size_t)a.last_total * 3 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  UAVMP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return UAVMP_OK;
+}
+
+// RRTStar::search, then the reference node's minimum-jerk step (test_minimum_jerk.cpp:40-75) for every query that reached the goal
+// with an optimal path of n >= 2 points: S = n - 1, one 1-D QP per axis, solved as ONE ragged batch (qp_solve_ragged_dev) whose
+// inputs are written on the device from the staged paths.  Query k of the QP set = problems 3k .. 3k+2, so its coefficients come out
+// axis-major [3][(order+1) S] and contiguous: the ragged coefficient array IS the per-query output.
+long long rrt_plan_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* start_vel, const double* end_pt, const uint64_t* query_seed,
+                         int order, double seg_time, const uavmp_osqp_settings* settings, int* search_status, int* n_segments,
+                         int* qp_solved, long long* coef_offsets, int* osqp_status, int* iters) {
+  cudaStream_t st = ctx->stream;
+  if (ctx->rrt) ctx->rrt->plan_total = -1;
+  cudaEventRecord(ctx->ev[0], st);
+  const long long total = rrt_search_run(ctx, B, start_pt, end_pt, query_seed);
+  if (total < 0) return total;
+  RrtState& a = *ctx->rrt;
+  cudaEventRecord(ctx->ev[1], st);
+  std::vector<int> nopt(B);
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(search_status, a.d_status, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  UAVMP_CUDA(ctx, cudaMemcpyAsync(nopt.data(), a.d_nopt, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, st));
+  UAVMP_CUDA(ctx, cudaStreamSynchronize(st));
+  // the QP set: REACH_END with at least two optimal-path points (the node would otherwise reuse a stale / empty path)
+  std::vector<long long> kq;
+  std::vector<int> Sp;
+  long long Q = 0;
+  for (int q = 0; q < B; q++) {
+    const int S = (search_status[q] == UAVMP_REACH_END && nopt[q] >= 2) ? nopt[q] - 1 : 0;
+    n_segments[q] = S;
+    if (!S) continue;
+    kq.push_back(q); kq.push_back(S); kq.push_back(Q);
+    for (int ax = 0; ax < 3; ax++) Sp.push_back(S);
+    Q += S;
+  }
+  const int M = (int)(kq.size() / 3), P = 3 * M, n1 = order + 1;
+  const long long sumS = 3 * Q;
+  // device: pos (sumS + P) | bv (2P) | ba = bj (2P, zero) | T (sumS) | coef (n1 sumS);  ints: solved | status | iters (P each)
+  const size_t o_bv = (size_t)(sumS + P), o_ba = o_bv + 2 * (size_t)P, o_T = o_ba + 2 * (size_t)P, o_coef = o_T + (size_t)sumS;
+  int qp_l = 0, aux_l = 0;
+  std::vector<int> pint(3 * (size_t)P);
+  if (M > 0) {
+    int r = ensure_bytes(ctx, (void**)&a.d_plan, &a.plan_bytes, (o_coef + (size_t)n1 * sumS) * sizeof(double)); if (r) return r;
+    r = ensure_bytes(ctx, (void**)&a.d_plan_i, &a.plan_i_bytes, 3 * (size_t)P * sizeof(int)); if (r) return r;
+    r = ensure_bytes(ctx, (void**)&a.d_plan_q, &a.plan_q_bytes, kq.size() * sizeof(long long)); if (r) return r;
+    std::vector<double> bv(2 * (size_t)P, 0.0);
+    for (int k = 0; k < M; k++)
+      for (int ax = 0; ax < 3; ax++) bv[2 * (3 * (size_t)k + ax)] = start_vel ? start_vel[3 * kq[3 * k] + ax] : 0.0;
+    double* d = a.d_plan;
+    UAVMP_CUDA(ctx, cudaMemcpyAsync(a.d_plan_q, kq.data(), kq.size() * sizeof(long long), cudaMemcpyHostToDevice, st));
+    UAVMP_CUDA(ctx, cudaMemcpyAsync(d + o_bv, bv.data(), bv.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    UAVMP_CUDA(ctx, cudaMemsetAsync(d + o_ba, 0, 2 * (size_t)P * sizeof(double), st));
+    k_rrt_plan_inputs<<<M, 128, 0, st>>>(a.d_plan_q, a.d_path_stage, a.path_cap, seg_time, d, d + o_T);
+    UAVMP_CUDA(ctx, cudaGetLastError());
+    cudaEventRecord(ctx->ev[2], st);
+    QpRaggedIo io;
+    io.pos = d; io.bv = d + o_bv; io.ba = d + o_ba; io.bj = d + o_ba; io.T = d + o_T;
+    io.coef = d + o_coef; io.solved = a.d_plan_i; io.status = a.d_plan_i + P; io.iters = a.d_plan_i + 2 * P; io.seg_off = nullptr;
+    io.order = order;
+    r = qp_solve_ragged_dev(ctx, st, ctx->qp_scr, order, P, Sp.data(), io, settings, &qp_l, &aux_l, nullptr, nullptr);
+    if (r) return r;
+    cudaEventRecord(ctx->ev[3], st);
+    UAVMP_CUDA(ctx, cudaMemcpyAsync(pint.data(), a.d_plan_i, pint.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
+    cudaEventRecord(ctx->ev[4], st);
+    UAVMP_CUDA(ctx, cudaStreamSynchronize(st));
+    a.d_plan_coef = d + o_coef;
+  }
+  // per-query outputs
+  long long off = 0;
+  int k = 0;
+  for (int q = 0; q < B; q++) {
+    if (coef_offsets) coef_offsets[q] = off;
+    int ok = 0;
+    for (int ax = 0; ax < 3; ax++) {
+      if (osqp_status) osqp_status[3 * q + ax] = 0;
+      if (iters) iters[3 * q + ax] = 0;
+    }
+    if (n_segments[q]) {
+      ok = 1;
+      for (int ax = 0; ax < 3; ax++) {
+        const int p = 3 * k + ax;
+        ok &= pint[p];
+        if (osqp_status) osqp_status[3 * q + ax] = pint[P + p];
+        if (iters) iters[3 * q + ax] = pint[2 * P + p];
+      }
+      off += 3 * (long long)n1 * n_segments[q];
+      k++;
+    }
+    qp_solved[q] = ok;
+  }
+  if (coef_offsets) coef_offsets[B] = off;
+  a.plan_total = off;
+  uavmp_timings& t = ctx->tm;
+  memset(&t, 0, sizeof(t));
+  cudaEventElapsedTime(&t.search_ms, ctx->ev[0], ctx->ev[1]);
+  if (M > 0) {
+    cudaEventElapsedTime(&t.path_ms, ctx->ev[1], ctx->ev[2]);
+    cudaEventElapsedTime(&t.qp_ms, ctx->ev[2], ctx->ev[3]);
+    cudaEventElapsedTime(&t.d2h_ms, ctx->ev[3], ctx->ev[4]);
+    cudaEventElapsedTime(&t.total_ms, ctx->ev[0], ctx->ev[4]);
+  } else {
+    t.total_ms = t.search_ms;
+  }
+  t.search_launches = 1; t.qp_launches = qp_l; t.aux_launches = 1 + (total > 0 ? 1 : 0) + (M > 0 ? 1 : 0) + aux_l;
+  return off;
+}
+
+int rrt_plan_get_coef(uavmp_ctx* ctx, double* coef, long long cap) {
+  if (!ctx->rrt || ctx->rrt->plan_total < 0) return uavmp_fail(ctx, UAVMP_ESTATE, "no uavmp_rrt_plan_batch call has completed");
+  RrtState& a = *ctx->rrt;
+  if (cap < a.plan_total) return uavmp_fail(ctx, UAVMP_ECAP, "coefficient buffer too small (%lld < %lld)", cap, a.plan_total);
+  if (a.plan_total > 0)
+    UAVMP_CUDA(ctx, cudaMemcpyAsync(coef, a.d_plan_coef, (size_t)a.plan_total * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   UAVMP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return UAVMP_OK;
 }

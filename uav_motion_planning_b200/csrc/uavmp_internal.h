@@ -134,6 +134,18 @@ struct RrtState;    // rrt_kernel.cu
 // device scratch of the stand-alone QP kernels (one per user of qp_solve_batch_dev: the context and every slot)
 struct QpScratch {
   void* ws = nullptr; size_t ws_bytes = 0;       // batch-interleaved workspace of the thread-per-problem kernel
+  void* tab = nullptr; size_t tab_bytes = 0;     // ragged batches: chunk counter | group table | segment offsets | problem ids
+  void* tmp = nullptr; size_t tmp_bytes = 0;     // ragged batches: contiguous copy of one thread-kernel group (inputs, outputs)
+};
+
+// One ragged batch of 1-D problems (qp_solve_ragged_dev): problem p has S_p segments; with so_p = sum_{i<p} S_i its waypoints start
+// at pos[so_p + p], its segment times at T[so_p], its coefficients at coef[(order + 1) so_p]; bv / ba / bj (B x 2) and the per-problem
+// outputs are indexed by p.  seg_off (so_p, device) is filled in by qp_solve_ragged_dev.
+struct QpRaggedIo {
+  const double *pos, *bv, *ba, *bj, *T;
+  double* coef; int *solved, *status, *iters;
+  const long long* seg_off;
+  int order;
 };
 
 // Everything ONE batch in flight owns.  Slot 0 runs on the context's stream and serves the synchronous entry points.
@@ -270,5 +282,13 @@ void astar_destroy(uavmp_ctx* ctx);
 long long rrt_search_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* end_pt, const uint64_t* query_seed, int* status,
                            int* use_node_num, long long* n_samples, double* goal_g_cost, uint64_t* tree_digest, long long* path_offsets);
 int rrt_get_paths(uavmp_ctx* ctx, double* path_xyz, long long cap_points);
+long long rrt_plan_batch(uavmp_ctx* ctx, int B, const double* start_pt, const double* start_vel, const double* end_pt, const uint64_t* query_seed,
+                         int order, double seg_time, const uavmp_osqp_settings* settings, int* search_status, int* n_segments,
+                         int* qp_solved, long long* coef_offsets, int* osqp_status, int* iters);
+int rrt_plan_get_coef(uavmp_ctx* ctx, double* coef, long long cap);
+// qp_kernel.cu: B problems with S_host[p] segments each (order 5 / 7, no corridor rows) in one grouped launch plus one thread-kernel
+// launch per S whose warp workspace does not fit in shared memory; asynchronous on `st`
+int qp_solve_ragged_dev(uavmp_ctx* ctx, cudaStream_t st, QpScratch& scr, int order, int B, const int* S_host, QpRaggedIo r,
+                        const uavmp_osqp_settings* settings, int* qp_launches, int* aux_launches, int* n_groups, int* n_thread_groups);
 void rrt_destroy(uavmp_ctx* ctx);
 uint32_t rrt_sample_seed_host(unsigned long long query_seed, long long i);

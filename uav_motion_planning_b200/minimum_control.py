@@ -58,6 +58,37 @@ class MinimumControl:
         self.last = dict(coef=coef, solved=solved, status=status, iters=iters)
         return self.last
 
+    def solve_batch_ragged(self, pos_1d, bound_vel, bound_acc, time_vec, S=None, bound_jerk=None, order=None, settings=None):
+        """B problems with a different number of segments each, one call (uavmp_minctrl_solve_ragged_batch).  Either lists (pos_1d[b]:
+        S_b + 1 waypoints, time_vec[b]: S_b times; S=None) or packed arrays plus S (B segment counts, problems in order).  bound_vel /
+        bound_acc (/ bound_jerk): B x 2.  Returns packed coef with coef_offsets (B + 1, problem b's coefficients are
+        coef[coef_offsets[b]:coef_offsets[b + 1]], segment-major as in solve_batch), solved, status, iters, S.  Every result is
+        bit-identical to solve_batch on that problem alone."""
+        order = self.order if order is None else order
+        if S is None:
+            S = np.array([len(t) for t in time_vec], np.int32)
+            pos = _lib.as_f64(np.concatenate([np.asarray(p, np.float64).reshape(-1) for p in pos_1d]))
+            T = _lib.as_f64(np.concatenate([np.asarray(t, np.float64).reshape(-1) for t in time_vec]))
+        else:
+            S = np.ascontiguousarray(S, np.int32).reshape(-1)
+            pos, T = _lib.as_f64(pos_1d).reshape(-1), _lib.as_f64(time_vec).reshape(-1)
+        B = len(S)
+        if pos.size != int(S.sum()) + B or T.size != int(S.sum()):
+            raise ValueError("pos_1d needs sum(S + 1) waypoints and time_vec sum(S) segment times")
+        bv = _lib.as_f64(bound_vel).reshape(B, 2)
+        ba = _lib.as_f64(bound_acc).reshape(B, 2)
+        bj = None if order == 5 else _lib.as_f64(np.zeros((B, 2)) if bound_jerk is None else bound_jerk).reshape(B, 2)
+        coef_offsets = np.zeros(B + 1, np.int64)
+        coef_offsets[1:] = np.cumsum(S.astype(np.int64) * (order + 1))
+        coef = np.zeros(int(coef_offsets[-1]))
+        solved, status, iters = np.zeros(B, np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32)
+        st = settings or self.settings
+        self.ctx.check(self.lib.uavmp_minctrl_solve_ragged_batch(
+            self.ctx.h, order, B, _lib.ptr(S), _lib.ptr(pos), _lib.ptr(bv), _lib.ptr(ba), _lib.ptr(bj), _lib.ptr(T), C.byref(st),
+            _lib.ptr(coef), _lib.ptr(solved), _lib.ptr(status), _lib.ptr(iters)))
+        self.last = dict(coef=coef, coef_offsets=coef_offsets, solved=solved, status=status, iters=iters, S=S)
+        return self.last
+
     # bool solve(VectorXd& pos_1d, Vector2d& bound_vel, Vector2d& bound_acc, VectorXd& time_vec)
     def solve(self, pos_1d, bound_vel, bound_acc, time_vec):
         r = self.solve_batch(np.asarray(pos_1d)[None], np.asarray(bound_vel)[None], np.asarray(bound_acc)[None],

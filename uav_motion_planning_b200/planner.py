@@ -140,3 +140,33 @@ def rrt_minimum_jerk_batch(rrt, optimizer, start_pt, end_pt, query_seed, start_v
             out[q] = dict(S=S, coef=res["coef"][3 * i:3 * i + 3].copy(), solved=res["solved"][3 * i:3 * i + 3].copy(),
                           iters=res["iters"][3 * i:3 * i + 3].copy())
     return r, out
+
+
+def rrt_plan_batch(rrt, start_pt, end_pt, query_seed, start_vel=None, order=5, seg_time=1.0, settings=None):
+    """The same flow as rrt_minimum_jerk_batch in ONE call (uavmp_rrt_plan_batch): the search, the QP inputs written on the device from
+    the optimal paths, and every query's three QPs in one ragged batch whatever their S.  Returns (raw, plans): raw = the packed
+    arrays (search_status, n_segments, qp_solved, coef_offsets, osqp_status[B, 3], iters[B, 3], coef); plans = one entry per query as
+    rrt_minimum_jerk_batch returns them, None or dict(S, coef[3, (order+1) S], solved[3], iters[3]).  rrt.search_batch-style paths
+    stay available through uavmp_rrt_get_paths."""
+    ctx = rrt.ctx
+    sp, ep = (_lib.as_f64(a).reshape(-1, 3) for a in (start_pt, end_pt))
+    B = sp.shape[0]
+    sv = None if start_vel is None else _lib.as_f64(start_vel).reshape(B, 3)
+    seeds = np.ascontiguousarray(np.broadcast_to(np.asarray(query_seed, np.uint64), (B,)))
+    status, nseg, solved = np.zeros(B, np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32)
+    offs = np.zeros(B + 1, np.int64)
+    ost, its = np.zeros((B, 3), np.int32), np.zeros((B, 3), np.int32)
+    total = ctx.check(ctx.lib.uavmp_rrt_plan_batch(ctx.h, B, _lib.ptr(sp), _lib.ptr(sv), _lib.ptr(ep), _lib.ptr(seeds), int(order),
+                                                   float(seg_time), C.byref(settings) if settings is not None else None,
+                                                   _lib.ptr(status), _lib.ptr(nseg), _lib.ptr(solved), _lib.ptr(offs), _lib.ptr(ost),
+                                                   _lib.ptr(its)))
+    coef = np.zeros(max(total, 1))
+    ctx.check(ctx.lib.uavmp_rrt_plan_get_coef(ctx.h, _lib.ptr(coef), max(total, 1)))
+    coef = coef[:total]
+    raw = dict(search_status=status, n_segments=nseg, qp_solved=solved, coef_offsets=offs, osqp_status=ost, iters=its, coef=coef)
+    n1 = order + 1
+    plans = [None if nseg[q] == 0 else
+             dict(S=int(nseg[q]), coef=coef[offs[q]:offs[q + 1]].reshape(3, n1 * nseg[q]).copy(),
+                  solved=(ost[q] == 1).astype(np.int32), iters=its[q].copy())
+             for q in range(B)]
+    return raw, plans
